@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- denoising-UNet frames/sec of the CamAnimate denoising path on B200 (BASELINE.json configs 2-5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (SURVEY.md 8d); default: config 2 on one GPU, config 4 under N > 1:
@@ -13,6 +13,8 @@ Workloads (SURVEY.md 8d); default: config 2 on one GPU, config 4 under N > 1:
 A "step" is one per-timestep pass of the hot path for the clip(s): configs 2-4 one UNet3DConditionModel.forward on the
 CFG-doubled batch; config 5 the three window forwards plus the on-device accumulate / CFG / DDIM glue.
 value = frames of all clips / t_step.
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float32); the inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 
   native arm     humanvid_b200 (hand-written sm_100a CUDA through the C ABI).  `value`: inputs resident in HBM, device time (CUDA
                  events) of K back-to-back steps, max over ranks.  `e2e`: the public Python call with the step's latents copied from
@@ -127,6 +129,21 @@ class ClockSampler:
                 "samples": len(self.rows)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each tensor as dirname/<name>.npy in float32.  Every bench workload returns a few MB, well inside DUMP_LIMIT_BYTES."""
+    import numpy as np
+
+    total = sum(a.numel() * 4 for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------ reference / CPU arm
 def cpu_threads():
     """Pinned (not probed) thread count for the CPU arm, so that repeated runs time the same thing: the CPUs this process may use
@@ -171,7 +188,7 @@ def cpu_reference_sample(cfg, samples=3, warmup=1, frames=2, cfg_batch=2):
     with torch.no_grad():
         for i in range(warmup + samples):
             t0 = time.perf_counter()
-            m(x, torch.tensor(500), ehs, pose_cond_fea=pose)
+            y = m(x, torch.tensor(500), ehs, pose_cond_fea=pose)[0]
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
@@ -180,7 +197,7 @@ def cpu_reference_sample(cfg, samples=3, warmup=1, frames=2, cfg_batch=2):
     # the step's windows overlap, so the clip's frames cost windows * fw * 2 passes per step
     passes_per_step = 2 * cfg["fw"] * cfg["windows"]
     fps = cfg["frames"] / (t * passes_per_step / passes)
-    return {"frames_per_s": fps, "s_per_sample": t, "cores": nthreads, "spread": (max(times) - min(times)) / t if len(times) > 1 else 0.0,
+    return {"output": y, "frames_per_s": fps, "s_per_sample": t, "cores": nthreads, "spread": (max(times) - min(times)) / t if len(times) > 1 else 0.0,
             "sample": f"oracle UNet forward (fp32, {nthreads} threads pinned by rule, denormals flushed) on {passes} of the step's {passes_per_step} "
                       f"frame-passes ({frames} frames x {cfg_batch} CFG halves) at the full {H}x{W} latent{' with the 16 reference banks' if cfg['banks'] else ''}; "
                       f"median of {len(times)} timed samples after {warmup} warm-up: {t:.1f} s (min {min(times):.1f}, max {max(times):.1f}); "
@@ -201,7 +218,9 @@ def workload_name(cfg, world):
 def run_reference(args, rank, cfg):
     if rank != 0:
         return
-    r = cpu_reference_sample(cfg, samples=max(1, min(args.steps, 3)), warmup=min(max(args.warmup, 0), 1))
+    r = cpu_reference_sample(cfg, samples=args.steps, warmup=min(max(args.warmup, 0), 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"noise_pred": r["output"]})
     line = {"metric": "denoising-UNet frames/sec, 24x768x576, CFG", "value": r["frames_per_s"], "unit": "frames/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000.0 * cfg["frames"] / r["frames_per_s"], "higher_is_better": True,
             "scaling": "strong" if cfg["name"] == "config5" else "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
@@ -542,6 +561,12 @@ def run_native(args, rank, world, local_rank, cfg):
         barrier()
     ms = e0.elapsed_time(e1) / args.steps
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:
+        # now, before the end-to-end loop below runs the same step again into the same buffers
+        dumped = {"latents": out} if is5 else {"noise_pred": out}
+        if world > 1 and not is5:
+            dumped["gathered_noise_pred_cond"] = gathered
+        dump_outputs(args.dump_outputs, dumped)
 
     # ---- end to end: the step's latents come from pinned host memory, the result goes back to the host
     src = loop.latents if is5 else sample
@@ -684,7 +709,10 @@ def main():
     ap.add_argument("--no-eager", action="store_true", help="skip the fp16-eager oracle timing on the GPU")
     ap.add_argument("--quick-cpu", action="store_true", help="2 instead of 3 timed CPU samples")
     ap.add_argument("--no-extras", action="store_true", help="skip the conditioning-branch timings and the 25-step pipeline clip")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -150,6 +150,18 @@ def make_writer(chs, xdim, seed=17):
     return ora, nat.to("cuda", torch.float16)
 
 
+def reference_banks_fp32(g):
+    """The writer's 16 banks in fp32 on the CPU: the golden file stores only a sample of them, and the oracle's fp32 CPU writer
+    reproduces the reference's banks (tests/test_oracle_cpu.py pins it against that sample at 1e-5)."""
+    w = O.synthetic_init(O.UNet2DConditionModel(block_out_channels=(64, 128, 256, 256), cross_attention_dim=64).eval(), seed=g["seed"])
+    O.set_reference_write(w)
+    with torch.no_grad():
+        w(g["lat"], torch.tensor(0), g["ehs"])
+    banks = O.written_banks(w)
+    assert all(torch.allclose(b[:, r], gb, atol=1e-5, rtol=1e-5) for b, r, gb in zip(banks, g["bank_rows"], g["bank_samples"]))
+    return banks
+
+
 def test_reference_writer_unet2d_golden_banks_and_chain():
     """Native reference ("writer") UNet: hidden + 16 banks against vectors from the reference's own UNet2DConditionModel in write
     mode; then writer -> ReferenceAttentionControl.update -> native denoising UNet against the reference's chain."""
@@ -162,9 +174,10 @@ def test_reference_writer_unet2d_golden_banks_and_chain():
         hid16 = ora.half()(lat, torch.tensor(0, device="cuda"), ehs)[0]
         ora.float()
     banks = [b.bank[0] for b, _ in nat.writer_blocks()]
-    assert hid.shape == (2, 64, 16, 16) and [tuple(b.shape) for b in banks] == [tuple(b.shape) for b in g["banks"]]
+    assert hid.shape == (2, 64, 16, 16) and [tuple(b.shape) for b in banks] == [tuple(s) for s in g["bank_shapes"]]
     e_hid, e_ref = rel(hid, g["hidden"].cuda()), rel(hid16, g["hidden"].cuda())
-    e_banks = [rel(b, gb.cuda()) for b, gb in zip(banks, g["banks"])]
+    # the golden file keeps a fixed, seeded quarter of every bank's tokens
+    e_banks = [rel(b[:, r.cuda()], gb.cuda()) for b, r, gb in zip(banks, g["bank_rows"], g["bank_samples"])]
     report(f"writer UNet2D: hidden native vs reference golden {e_hid:.2e} (fp16-eager {e_ref:.2e}); banks max {max(e_banks):.2e}")
     assert e_hid <= e_ref + 2e-4
     assert max(e_banks) <= 2e-3
@@ -175,7 +188,7 @@ def test_reference_writer_unet2d_golden_banks_and_chain():
     x3 = g["x3"].cuda().half()
     with torch.no_grad():
         y = nat3(x3, g["t3"], ehs, return_dict=False)[0]
-        O.set_reference_banks(ora3, [gb.cuda().half() for gb in g["banks"]], cfg=True)
+        O.set_reference_banks(ora3, [gb.cuda().half() for gb in reference_banks_fp32(g)], cfg=True)
         y16 = ora3.half()(x3, torch.tensor(g["t3"], device="cuda"), ehs)[0]
     e_nat, e_16 = rel(y, g["y3"].cuda()), rel(y16, g["y3"].cuda())
     report(f"writer -> reader chain: native vs reference golden {e_nat:.2e} (fp16-eager {e_16:.2e})")

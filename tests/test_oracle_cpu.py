@@ -68,8 +68,9 @@ def test_reference_writer_unet2d_golden_and_chain():
         hid = w(g["lat"], torch.tensor(0), g["ehs"])[0]
     banks = O.written_banks(w)
     assert torch.allclose(hid, g["hidden"], atol=1e-5, rtol=1e-5)
-    assert len(banks) == 16 and [tuple(b.shape) for b in banks] == [tuple(b.shape) for b in g["banks"]]
-    assert all(torch.allclose(a, b, atol=1e-5, rtol=1e-5) for a, b in zip(banks, g["banks"]))
+    assert len(banks) == 16 and [tuple(b.shape) for b in banks] == [tuple(s) for s in g["bank_shapes"]]
+    # the golden file keeps a fixed, seeded quarter of every bank's tokens
+    assert all(torch.allclose(a[:, r], b, atol=1e-5, rtol=1e-5) for a, r, b in zip(banks, g["bank_rows"], g["bank_samples"]))
     # a bank is LayerNorm-1's output: zero mean / unit variance per token for the synthetic affine-free init is not assumed; only shape + order
     assert [b.shape[2] for b in banks] == [256] * 6 + [128] * 5 + [64] * 5 and banks[5].shape[1] == 4
     r = O.synthetic_init(O.UNet3DConditionModel(block_out_channels=(64, 128, 256, 256), cross_attention_dim=64).eval(), seed=g["seed3"])
